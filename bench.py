@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py — Mbases/s depth-counted on a synthetic 30x WGS-shaped alignment stream (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload wgs|chr20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload wgs|chr20] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR : after the timed steps, rank 0 repeats one step of `value` and one of `e2e` untimed and writes what a
+        caller of those paths receives as DIR/*.npy (float64, or float32 for text bytes; under 64 MB): window sums and
+        class runs of every contig, and the BED text lengths plus a seeded sample of the text.  The workload is seeded, so
+        two builds run with the same arguments can be compared output for output.
 
 Workload (default, every N): BASELINE configs[2], the 25 primary GRCh38 contigs (3,088,286,401 bp) at 30x / 150 bp
 reads, W=500 — STRONG scaling: the same genome at every N, contigs dealt to the ranks longest-first (gl_lpt_assign, the
@@ -169,13 +174,11 @@ def run_reference(args):
     total = sum(c[1] for c in contigs)
     nseg = sum(c[2].size for c in contigs)
     log(f"[reference] synth: {nseg} segments over {total} bp in {time.time() - t0:.1f}s; {threads} threads")
-    times, chunks, budget0 = [], 0, time.time()
+    times, chunks = [], 0
     for i in range(args.warmup + args.steps):
         dt, _, chunks = cpu_genome_pass(orc, contigs, threads)
         if i >= args.warmup:
             times.append(dt)
-        if times and time.time() - budget0 > 150:            # bounded: stop after ~2.5 min with at least one timed step
-            break
     t = float(np.mean(times))
     val = total / t / 1e6
     out = {"impl": "reference", "metric": METRIC, "value": val, "unit": "Mbases/s", "n_gpus": args.gpus,
@@ -561,6 +564,40 @@ def cli_wallclock(n_cpus):
         shutil.rmtree(tmp, ignore_errors=True)
 
 
+DUMP_TEXT_SAMPLE = 1 << 20           # bytes of each BED text kept by --dump-outputs (a seeded sample when the text is longer)
+DUMP_MAX_WINDOWS = 6_500_000         # float64 window sums kept (the whole 25-contig genome has 6,176,584 windows at W=500)
+DUMP_MAX_RUNS = 100_000
+
+
+def fixed_sample(a, cap, seed):
+    """a itself when it has at most cap elements, else cap elements at seeded positions (in order)"""
+    if a.size <= cap:
+        return a
+    return a[np.sort(np.random.default_rng(seed).integers(0, a.size, cap))]
+
+
+def dump_outputs(out_dir, resident, texts):
+    """resident: per contig (window sums, run starts, run classes) of the resident step; texts: per contig (.depth.bed,
+    .callable.bed) bytes of the drop-in call.  Writes out_dir/*.npy; integers are exact in float64."""
+    def text_sample(parts, seed):
+        return fixed_sample(np.frombuffer(b"".join(parts), np.uint8), DUMP_TEXT_SAMPLE, seed).astype(np.float32)
+    arrays = {
+        "depth_contig_sizes": np.array([(ws.size, rs.size) for ws, rs, _ in resident], np.float64),
+        "depth_window_sum": fixed_sample(np.concatenate([r[0] for r in resident]).astype(np.float64), DUMP_MAX_WINDOWS, 1),
+        "depth_run_start": fixed_sample(np.concatenate([r[1] for r in resident]).astype(np.float64), DUMP_MAX_RUNS, 2),
+        "depth_run_class": fixed_sample(np.concatenate([r[2] for r in resident]).astype(np.float64), DUMP_MAX_RUNS, 2),
+        "e2e_text_lengths": np.array([(len(h), len(c)) for h, c in texts], np.float64),
+        "e2e_depth_bed_bytes": text_sample([t[0] for t in texts], 3),
+        "e2e_callable_bed_bytes": text_sample([t[1] for t in texts], 4),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[dump] {len(arrays)} arrays, {total} bytes -> {out_dir}")
+
+
 # ------------------------------------------------------------------------------------------------ GPU arm
 def main():
     ap = argparse.ArgumentParser()
@@ -571,7 +608,12 @@ def main():
     ap.add_argument("--workload", default=os.environ.get("GL_BENCH_WORKLOAD", "wgs"), choices=["wgs", "chr20"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the per-path extras (int32 / general path / packed e2e variants)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed paths as DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -636,11 +678,13 @@ def main():
         if dist is not None:
             dist.barrier()
 
-    def step_resident():
+    def step_resident(keep=None):
         for w in work:
             ctx.depth_begin(0, w["L"])
             ctx.depth_add_segments_packed8_device(w["d_a"], w["d_d"], w["d_l"], w["nb"])
             ctx.depth_reduce(W, MINCOV, MAXMEAN, STEP)
+            if keep is not None:
+                keep.append((ctx.depth_get_windows(),) + ctx.depth_get_runs())
 
     text_bytes = [0, 0]
     tr = {"h2d": 0, "pack_s": 0.0, "escaped": 0, "paths": set(), "kinds": set()}
@@ -659,13 +703,15 @@ def main():
         lanes[k]["work"].append(w); lane_load[k] += w["nseg"]
     lane_pool = ThreadPoolExecutor(max_workers=2)
 
-    def run_lane(lane):
+    def run_lane(lane, keep=None):
         c, o = lane["ctx"], lane["o"]
         hb = cb = 0
         h2d, pack_s, esc = 0, 0.0, 0
         kinds, paths = set(), set()
         for w in lane["work"]:
             hl, cl = c.depth_bed_contig(w["name"], w["L"], w["h_s"], w["h_e"], W, MINCOV, MAXMEAN, STEP, threads=0, out=o, raw=True)
+            if keep is not None:
+                keep.append((bytes(o[0][:hl]), bytes(o[1][:cl])))
             hb += hl; cb += cl
             kind, ps, nb, ne = c.depth_transport_stats()
             h2d += nb; pack_s += ps; esc += ne
@@ -759,6 +805,11 @@ def main():
         ms_e2e_one_lane += (time.perf_counter() - te0) * 1e3
     ms_e2e_one_lane /= n_one
     barrier()
+    if args.dump_outputs and rank == 0:
+        resident, texts = [], []
+        step_resident(resident)
+        run_lane({"ctx": ctx, "o": (o_hd, o_ca), "work": work}, texts)
+        dump_outputs(args.dump_outputs, resident, texts)
 
     # ---- per-kernel live timing for the roofline: CUDA events on the launching stream around every kernel of the same
     #      step (library-side, gl_profile_*), averaged over the repetitions
